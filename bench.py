@@ -78,7 +78,39 @@ def parse():
     ap.add_argument("--no-graph-cache", action="store_true", help="always rebuild the HNSW graph (default: reuse /tmp/tsgpu_bench_cache)")
     ap.add_argument("--exp-sorted-vectors", action="store_true",
                     help="experiment only: store vectors in cluster order (seq_id locality) to measure what row locality is worth")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the results of the last timed step to DIR/<name>.npy (see dump_outputs)")
     return ap.parse_args()
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, kv, cnt, found):
+    """The results a caller of the timed path receives for its last step: per query its hit count and found count, per hit the
+    fields of the KV record. Every array is float64 (vector_distance stays float32); int64 fields are split into exact high
+    (signed) and low 32-bit halves, and records past a query's count are zeroed. Above DUMP_LIMIT bytes in all, a fixed, seeded
+    sample of the queries is written; query_rows.npy names the rows written, in order."""
+    nq, stride = kv.shape
+    cnt = np.asarray(cnt, np.int64)
+    kv = np.ascontiguousarray(kv).copy()
+    kv.view(np.uint8).reshape(nq, stride, kv.dtype.itemsize)[np.arange(stride)[None, :] >= cnt[:, None]] = 0
+    per_query = stride * 13 * 8 + 3 * 8
+    rows = np.arange(nq)
+    if nq * per_query > DUMP_LIMIT:
+        rows = np.sort(np.random.default_rng(0).choice(nq, DUMP_LIMIT // per_query, replace=False))
+    kv = kv[rows]
+    f64 = lambda a: np.asarray(a, np.float64)
+    arrays = {"query_rows": f64(rows), "count": f64(cnt[rows]), "found": f64(np.asarray(found)[rows]),
+              "key": f64(kv["key"]), "distinct_key": f64(kv["distinct_key"]),
+              "scores_hi": f64(kv["scores"] >> 32), "scores_lo": f64(kv["scores"] & 0xFFFFFFFF),
+              "text_match_score_hi": f64(kv["text_match_score"] >> 32), "text_match_score_lo": f64(kv["text_match_score"] & 0xFFFFFFFF),
+              "vector_distance": np.asarray(kv["vector_distance"], np.float32), "match_score_index": f64(kv["match_score_index"]),
+              "query_index": f64(kv["query_index"])}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"outputs of the last timed step: {len(rows)} of {nq} queries, {sum(a.nbytes for a in arrays.values()) / 1e6:.1f} MB in {out_dir}")
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -367,8 +399,11 @@ def run_reference(args, rank, world):
         step(i)
     t0 = time.perf_counter()
     for i in range(args.steps):
-        st = step(args.warmup + i)[3]
+        res = step(args.warmup + i)
     dt = time.perf_counter() - t0
+    st = res[3]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res[0], res[1], res[2])
     qps = S_n * args.steps / dt
     out = {"impl": "reference", "metric": "queries/sec", "value": qps, "unit": "queries/s", "n_gpus": args.gpus, "steps": args.steps,
            "warmup": args.warmup, "ms_per_step": 1000 * dt / args.steps, "higher_is_better": True, "scaling": SCALING,
@@ -663,6 +698,9 @@ def run_tsgpu(args, rank, world, local_rank):
         sampler.start()
     dt_res, sts = timed(0)
     launches = gi.stats()["launches_total"] - launches0
+    if args.dump_outputs and rank == 0:            # this rank's slice; copied before the later legs reuse the buffers
+        dump_outputs(args.dump_outputs, np.frombuffer(kv_dev[:nl * rec].cpu().numpy().tobytes(), S.KV_DTYPE).reshape(nl, stride),
+                     cnt_dev[:nl].cpu().numpy(), fnd_dev[:nl].cpu().numpy())
     dt_pin, sts_pin = timed(1)
     x0 = xfer()
     dt_e2e, sts_e2e = timed_e2e()

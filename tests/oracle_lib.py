@@ -6,6 +6,9 @@ Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline/--impl referenc
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import json
+import lzma
 import os
 import subprocess
 from typing import List, Optional, Sequence
@@ -97,6 +100,85 @@ def have_ref() -> bool:
     if not os.path.exists(REF_SO) and os.path.isdir("/root/reference/src"):
         build_oracle()
     return os.path.exists(REF_SO)
+
+
+REF_ANSWERS_DIR = os.path.join(ROOT, "tests", "golden", "ref_answers")
+
+
+def _plain(v):
+    if isinstance(v, np.ndarray):
+        return v.tolist()
+    if isinstance(v, (list, tuple)):
+        return [_plain(x) for x in v]
+    if isinstance(v, dict):
+        return {str(k): _plain(x) for k, x in v.items()}
+    if isinstance(v, np.generic):
+        return v.item()
+    return v
+
+
+class RefAnswers:
+    """What the reference's own compiled sources answered in one test, in call order, stored under
+    tests/golden/ref_answers/<group>.json.xz so the comparison runs where oracle/_ref cannot be built.
+
+    `ref(fn)` returns fn()'s answer as plain lists / numbers / strings; `ref.same(got, fn)` says whether `got` equals it, and
+    stores a long answer as a 128-bit SHA-256 digest only. With oracle/_ref built, fn runs and its answer must equal the stored one
+    (TSGPU_REF_RECORD=1 stores the live answers instead); without it, the stored answer is used and fn is not called, so fn
+    alone may touch ol.ref()."""
+
+    def __init__(self, group: str, name: str):
+        self.path = os.path.join(REF_ANSWERS_DIR, group + ".json.xz")
+        self.name = name
+        self.live = have_ref()
+        self.record = self.live and os.environ.get("TSGPU_REF_RECORD") == "1"
+        self.stored = _load_answers(self.path).get(name)
+        assert self.record or self.stored is not None, \
+            f"no stored reference answers for {group}/{name}: record them with TSGPU_REF_RECORD=1 where oracle/_ref is built"
+        self.got = []
+
+    def __call__(self, fn):
+        i = len(self.got)
+        if self.live:
+            v = _plain(fn())
+            if not self.record:
+                assert i < len(self.stored) and v == self.stored[i], f"{self.name}: reference answer {i} differs from the stored one"
+        else:
+            assert i < len(self.stored), f"{self.name}: more reference calls than stored answers"
+            v = self.stored[i]
+        self.got.append(v)
+        return v
+
+    def same(self, got, fn) -> bool:
+        return _compact(got) == self(lambda: _compact(fn()))
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, exc_type, exc, tb):
+        if exc_type is not None:
+            return False
+        if self.record:
+            data = _load_answers(self.path)
+            data[self.name] = self.got
+            os.makedirs(REF_ANSWERS_DIR, exist_ok=True)
+            with open(self.path, "wb") as f:
+                f.write(lzma.compress(json.dumps(data, sort_keys=True, separators=(",", ":")).encode(), preset=9 | lzma.PRESET_EXTREME))
+        else:
+            assert len(self.got) == len(self.stored), f"{self.name}: {len(self.got)} reference calls, {len(self.stored)} stored answers"
+        return False
+
+
+def _compact(v):
+    v = _plain(v)
+    s = json.dumps(v, sort_keys=True, separators=(",", ":"))
+    return v if len(s) <= 64 else "sha256:" + hashlib.sha256(s.encode()).hexdigest()[:32]
+
+
+def _load_answers(path: str) -> dict:
+    if not os.path.exists(path):
+        return {}
+    with open(path, "rb") as f:
+        return json.loads(lzma.decompress(f.read()))
 
 
 class RefParams(C.Structure):

@@ -3,7 +3,8 @@ oracle/_ref. A reference tree is filled with art_insert document by document (as
 (ref_art_export) and loaded into the mirror; art_fuzzy_search_i and art_mirror_t::fuzzy_search must then return the SAME
 tokens in the SAME order — typos 0..2, prefix and whole-word search, both token orders, max_words truncation, pre-excluded
 tokens, the previous-token restriction and a filter; ties included. A second check covers the mirror BUILT from a
-vocabulary (no live tree): same candidates up to the order of equal-score tokens."""
+vocabulary (no live tree): same candidates up to the order of equal-score tokens. Without oracle/_ref the reference's exported
+trees and answers come from tests/golden/ref_answers (oracle_lib.RefAnswers)."""
 import ctypes as C
 import os
 import subprocess
@@ -79,6 +80,15 @@ def export(R, t):
     return buf.raw
 
 
+def stored_export(ref, t):
+    """the reference tree's export, through the stored answers (hex text)"""
+    return bytes.fromhex(ref(lambda: export(ol.ref(), t).hex()))
+
+
+def ref_answers(name):
+    return ol.RefAnswers("test_art_mirror", name)
+
+
 def bind(am, h, coll):
     toks = sorted(coll.vocab, key=coll.vocab.get)
     lo = np.ascontiguousarray(coll.flat.list_off, np.uint64)
@@ -130,61 +140,64 @@ def run_am(am, h, q):
     return [x for x in buf.value.decode().split("\n") if x]
 
 
-@pytest.mark.skipif(not ol.have_ref() or not hasattr(ol.ref(), "ref_art_new"), reason="oracle/_ref with the reference's art.cpp not built")
 def test_loaded_mirror_returns_the_references_candidates_in_order(am):
-    R = ol.ref()
     rng = np.random.default_rng(77)
     n = hits = 0
-    for trial in range(48):
-        coll = make_collection(rng, trial)
-        t = ref_tree(R, coll)
-        blob = export(R, t)
-        h = am.am_load(blob, len(blob))
-        assert h, "export did not parse"
-        assert am.am_num_leaves(h) == len(coll.vocab)
-        keep = bind(am, h, coll)
-        for q in queries(rng, coll, 80):
-            want, got = run_ref(R, t, q), run_am(am, h, q)
-            assert got == want, (trial, {k: (v.tolist() if isinstance(v, np.ndarray) else v) for k, v in q.items()}, want, got)
-            n += 1
-            hits += len(want)
-        am.am_free(h)
-        R.ref_art_free(t)
-        del keep
+    with ref_answers("loaded_mirror") as ref:
+        for trial in range(48):
+            coll = make_collection(rng, trial)
+            t = ref_tree(ol.ref(), coll) if ref.live else None
+            blob = stored_export(ref, t)
+            h = am.am_load(blob, len(blob))
+            assert h, "export did not parse"
+            assert am.am_num_leaves(h) == len(coll.vocab)
+            keep = bind(am, h, coll)
+            for q in queries(rng, coll, 80):
+                got = run_am(am, h, q)
+                assert ref.same(got, lambda: run_ref(ol.ref(), t, q)), (trial, {k: (v.tolist() if isinstance(v, np.ndarray) else v) for k, v in q.items()}, got)
+                n += 1
+                hits += len(got)
+            am.am_free(h)
+            if ref.live:
+                ol.ref().ref_art_free(t)
+            del keep
     assert n > 3000 and hits > 4000, (n, hits)
 
 
-@pytest.mark.skipif(not ol.have_ref() or not hasattr(ol.ref(), "ref_art_new"), reason="oracle/_ref with the reference's art.cpp not built")
 def test_reference_fixture_tokens(am):
     """test/documents.jsonl (the collection_test.cpp fixture): prefix / typo candidates of the scenario queries."""
-    R = ol.ref()
     coll = refflow.Collection.from_jsonl(os.path.join(ROOT, "tests", "golden", "documents.jsonl"))
-    t = ref_tree(R, coll)
-    blob = export(R, t)
-    h = am.am_load(blob, len(blob))
-    keep = bind(am, h, coll)
-    for term, cost, prefix in [("loox", 1, 0), ("lau", 0, 1), ("launch", 0, 0), ("rocket", 1, 0), ("ro", 0, 1), ("t", 0, 1), ("kind", 1, 1),
-                               ("the", 0, 0), ("laun", 1, 1), ("ex", 0, 1), ("what", 0, 1), ("rokket", 2, 0), ("lauch", 1, 0)]:
-        for order in (0, 1):
-            q = dict(term=term, cost=cost, prefix=prefix, order=order, max_words=4, excl=[], prev="", filt=None)
-            assert run_am(am, h, q) == run_ref(R, t, q), q
-    q = dict(term="loox", cost=1, prefix=0, order=0, max_words=4, excl=[], prev="", filt=None)
-    assert run_ref(R, t, q) == ["look", "loop"]            # QueryWithTypo's candidates, most frequent first
-    am.am_free(h)
-    R.ref_art_free(t)
-    del keep
+    with ref_answers("fixture_tokens") as ref:
+        t = ref_tree(ol.ref(), coll) if ref.live else None
+        blob = stored_export(ref, t)
+        h = am.am_load(blob, len(blob))
+        keep = bind(am, h, coll)
+        for term, cost, prefix in [("loox", 1, 0), ("lau", 0, 1), ("launch", 0, 0), ("rocket", 1, 0), ("ro", 0, 1), ("t", 0, 1), ("kind", 1, 1),
+                                   ("the", 0, 0), ("laun", 1, 1), ("ex", 0, 1), ("what", 0, 1), ("rokket", 2, 0), ("lauch", 1, 0)]:
+            for order in (0, 1):
+                q = dict(term=term, cost=cost, prefix=prefix, order=order, max_words=4, excl=[], prev="", filt=None)
+                assert run_am(am, h, q) == ref(lambda: run_ref(ol.ref(), t, q)), q
+        q = dict(term="loox", cost=1, prefix=0, order=0, max_words=4, excl=[], prev="", filt=None)
+        assert ref(lambda: run_ref(ol.ref(), t, q)) == ["look", "loop"]            # QueryWithTypo's candidates, most frequent first
+        am.am_free(h)
+        if ref.live:
+            ol.ref().ref_art_free(t)
+        del keep
 
 
-@pytest.mark.skipif(not ol.have_ref() or not hasattr(ol.ref(), "ref_art_new"), reason="oracle/_ref with the reference's art.cpp not built")
 def test_built_mirror_matches_up_to_tie_order(am):
     """No live tree to export (this repository's harness): the mirror built from the vocabulary finds the same candidates;
     tokens of equal rank may come in another order (the reference's inner-node scores depend on its insertion history)."""
-    R = ol.ref()
+    with ref_answers("built_mirror") as ref:
+        _built_mirror_matches(am, ref)
+
+
+def _built_mirror_matches(am, ref):
     rng = np.random.default_rng(5)
     n = 0
     for trial in range(20):
         coll = make_collection(rng, trial)
-        t = ref_tree(R, coll)
+        t = ref_tree(ol.ref(), coll) if ref.live else None
         toks = sorted(coll.vocab, key=coll.vocab.get)
         fl = coll.flat
         df = np.diff(fl.list_off.astype(np.int64)).astype(np.uint32)
@@ -194,20 +207,33 @@ def test_built_mirror_matches_up_to_tie_order(am):
         rank = [dict(zip(toks, df.tolist())), dict(zip(toks, ms.tolist()))]
         for q in queries(rng, coll, 60):
             q["max_words"] = 100000               # truncation would make membership depend on the tie order
-            want, got = run_ref(R, t, q), run_am(am, h, q)
-            assert sorted(want) == sorted(got), (trial, q, want, got)
+            got = run_am(am, h, q)
+            assert ref.same(sorted(got), lambda: sorted(run_ref(ol.ref(), t, q))), (trial, q, got)
             exact_first = q["cost"] == 0 and q["term"] in coll.vocab and q["term"] not in q["excl"]
             body = got[1:] if exact_first and got and got[0] == q["term"] else got
             ranks = [rank[q["order"]][x] for x in body]
             assert ranks == sorted(ranks, reverse=True), (trial, q, got)
             n += 1
         am.am_free(h)
-        R.ref_art_free(t)
+        if ref.live:
+            ol.ref().ref_art_free(t)
         del keep
     assert n > 800
 
 
 # ---- the reference's own ART tests (test/art_test.cpp) with inline keys or the two small word lists it ships
+class _RefTree:
+    """a reference tree (live only) and its export (live or stored)"""
+
+    def __init__(self, ref, keys, scores=None):
+        self.t = _tree_of(ol.ref(), keys, scores) if ref.live else None
+        self.blob = stored_export(ref, self.t)
+
+    def free(self):
+        if self.t is not None:
+            ol.ref().ref_art_free(self.t)
+
+
 def _tree_of(R, keys, scores=None):
     """art_insert(key, get_document(id)): id = score = position (1-based) unless scores are given (art_test.cpp:18-21)."""
     t = R.ref_art_new()
@@ -218,102 +244,103 @@ def _tree_of(R, keys, scores=None):
     return t
 
 
-def _both(R, am, t, term, lo, hi, max_words, order, prefix):
-    blob = export(R, t)
-    h = am.am_load(blob, len(blob))
+def _both(ref, am, tree, term, lo, hi, max_words, order, prefix):
+    h = am.am_load(tree.blob, len(tree.blob))
     assert h
     tb = term if isinstance(term, bytes) else term.encode()
-    out = []
-    for fn, handle in ((R.ref_art_fuzzy, t), (None, h)):
+
+    def fuzzy(fn, handle, *rest):
         buf = C.create_string_buffer(1 << 16)
-        if fn is not None:
-            fn(handle, tb, lo, hi, max_words, order, prefix, 0, b"", None, 0, 0, b"", buf, len(buf))
-        else:
-            am.am_fuzzy(handle, tb, lo, hi, max_words, order, prefix, b"", None, 0, 0, b"", buf, len(buf))
-        out.append([x for x in buf.value.split(b"\n") if x])
+        fn(handle, tb, lo, hi, max_words, order, prefix, *rest, buf, len(buf))
+        return [x.decode() for x in buf.value.split(b"\n") if x]
+    want = ref(lambda: fuzzy(ol.ref().ref_art_fuzzy, tree.t, 0, b"", None, 0, 0, b""))
+    got = fuzzy(am.am_fuzzy, h, b"", None, 0, 0, b"")
     am.am_free(h)
-    assert out[0] == out[1], (term, lo, hi, out)
-    return [x.decode() for x in out[1]]
+    assert want == got, (term, lo, hi, want, got)
+    return got
 
 
-@pytest.mark.skipif(not ol.have_ref() or not hasattr(ol.ref(), "ref_art_new"), reason="oracle/_ref with the reference's art.cpp not built")
 def test_reference_art_tests(am):
-    R = ol.ref()
+    with ref_answers("reference_art_tests") as ref:
+        _reference_art_tests(am, ref)
+
+
+def _reference_art_tests(am, ref):
     FREQ, SCORE = 0, 1
     # test_art_fuzzy_search_single_leaf :579
-    t = _tree_of(R, ["implement"])
-    assert len(_both(R, am, t, "implement", 0, 0, 10, FREQ, 0)) == 1
-    assert len(_both(R, am, t, "implment", 0, 0, 10, FREQ, 0)) == 0
-    assert len(_both(R, am, t, "implment", 0, 1, 10, FREQ, 0)) == 1
-    assert len(_both(R, am, t, "implwnent", 0, 2, 10, FREQ, 0)) == 1
-    R.ref_art_free(t)
+    t = _RefTree(ref, ["implement"])
+    assert len(_both(ref, am, t, "implement", 0, 0, 10, FREQ, 0)) == 1
+    assert len(_both(ref, am, t, "implment", 0, 0, 10, FREQ, 0)) == 0
+    assert len(_both(ref, am, t, "implment", 0, 1, 10, FREQ, 0)) == 1
+    assert len(_both(ref, am, t, "implwnent", 0, 2, 10, FREQ, 0)) == 1
+    t.free()
     # test_art_fuzzy_search_single_leaf_prefix :617
-    t = _tree_of(R, ["application"])
-    assert len(_both(R, am, t, "aplication", 0, 1, 10, FREQ, 1)) == 1
-    assert len(_both(R, am, t, "aplication", 0, 2, 10, FREQ, 1)) == 1
-    R.ref_art_free(t)
+    t = _RefTree(ref, ["application"])
+    assert len(_both(ref, am, t, "aplication", 0, 1, 10, FREQ, 1)) == 1
+    assert len(_both(ref, am, t, "aplication", 0, 2, 10, FREQ, 1)) == 1
+    t.free()
     # ..._qlen_greater_than_key :643, ..._non_prefix :661, test_art_prefix_larger_than_key :684
-    t = _tree_of(R, ["storka"])
-    assert _both(R, am, t, "starkbin", 0, 2, 10, FREQ, 1) == []
-    R.ref_art_free(t)
-    t = _tree_of(R, ["spz005"])
-    assert _both(R, am, t, "spz", 0, 1, 10, FREQ, 0) == []
-    assert _both(R, am, t, "spz", 0, 1, 10, FREQ, 1) == ["spz005"]
-    R.ref_art_free(t)
-    t = _tree_of(R, ["arvin"])
-    assert _both(R, am, t, "earrings", 0, 2, 10, FREQ, 0) == []
-    R.ref_art_free(t)
+    t = _RefTree(ref, ["storka"])
+    assert _both(ref, am, t, "starkbin", 0, 2, 10, FREQ, 1) == []
+    t.free()
+    t = _RefTree(ref, ["spz005"])
+    assert _both(ref, am, t, "spz", 0, 1, 10, FREQ, 0) == []
+    assert _both(ref, am, t, "spz", 0, 1, 10, FREQ, 1) == ["spz005"]
+    t.free()
+    t = _RefTree(ref, ["arvin"])
+    assert _both(ref, am, t, "earrings", 0, 2, 10, FREQ, 0) == []
+    t.free()
     # test_art_fuzzy_search_prefix_token_ordering :702 — score = 12 - i; the exact token comes first
     keys = ["enter", "elephant", "enamel", "ercot", "enyzme", "energy", "epoch", "epyc", "express", "everest", "end", "e"]
-    t = _tree_of(R, keys, scores=[len(keys) - i for i in range(len(keys))])
-    assert _both(R, am, t, "e", 0, 0, 3, SCORE, 1) == ["e", "enter", "elephant"]
-    assert _both(R, am, t, "enter", 1, 1, 3, SCORE, 1) == []
-    R.ref_art_free(t)
+    t = _RefTree(ref, keys, scores=[len(keys) - i for i in range(len(keys))])
+    assert _both(ref, am, t, "e", 0, 0, 3, SCORE, 1) == ["e", "enter", "elephant"]
+    assert _both(ref, am, t, "enter", 1, 1, 3, SCORE, 1) == []
+    t.free()
     # test_art_fuzzy_search_unicode_chars :864
     keys = ["роман", "обладать", "роисхождения", "без", "பஞ்சமம்", "சுதந்திரமாகவே", "அல்லது", "அடிப்படையில்"]
-    t = _tree_of(R, keys)
+    t = _RefTree(ref, keys)
     for k in keys:
-        assert _both(R, am, t, k, 0, 0, 10, FREQ, 1) == [k]
-    R.ref_art_free(t)
+        assert _both(ref, am, t, k, 0, 0, 10, FREQ, 1) == [k]
+    t.free()
     # test_art_fuzzy_search_extra_chars :891, roche_chews :1083, raspberry :1118, highliving :1152, ill_like_tokens2 :1035
-    t = _tree_of(R, ["abbviation"])
-    assert len(_both(R, am, t, "abbreviation", 0, 2, 10, FREQ, 1)) == 1
-    R.ref_art_free(t)
-    t = _tree_of(R, ["roche"])
-    assert _both(R, am, t, "chews", 0, 2, 10, FREQ, 1) == []
-    assert _both(R, am, t, "roche", 0, 0, 10, FREQ, 0) == ["roche"]
-    assert _both(R, am, t, "xxroche", 0, 2, 10, FREQ, 0) == ["roche"]
-    R.ref_art_free(t)
-    t = _tree_of(R, ["raspberry", "raspberries"])
-    assert len(_both(R, am, t, "raspberries", 0, 2, 10, FREQ, 1)) == 2
-    assert len(_both(R, am, t, "raspberry", 0, 2, 10, FREQ, 1)) == 2
-    R.ref_art_free(t)
-    t = _tree_of(R, ["highliving"])
-    assert len(_both(R, am, t, "higghliving", 0, 1, 10, FREQ, 0)) == 1
-    assert len(_both(R, am, t, "higghliving", 0, 2, 10, FREQ, 1)) == 1
-    R.ref_art_free(t)
+    t = _RefTree(ref, ["abbviation"])
+    assert len(_both(ref, am, t, "abbreviation", 0, 2, 10, FREQ, 1)) == 1
+    t.free()
+    t = _RefTree(ref, ["roche"])
+    assert _both(ref, am, t, "chews", 0, 2, 10, FREQ, 1) == []
+    assert _both(ref, am, t, "roche", 0, 0, 10, FREQ, 0) == ["roche"]
+    assert _both(ref, am, t, "xxroche", 0, 2, 10, FREQ, 0) == ["roche"]
+    t.free()
+    t = _RefTree(ref, ["raspberry", "raspberries"])
+    assert len(_both(ref, am, t, "raspberries", 0, 2, 10, FREQ, 1)) == 2
+    assert len(_both(ref, am, t, "raspberry", 0, 2, 10, FREQ, 1)) == 2
+    t.free()
+    t = _RefTree(ref, ["highliving"])
+    assert len(_both(ref, am, t, "higghliving", 0, 1, 10, FREQ, 0)) == 1
+    assert len(_both(ref, am, t, "higghliving", 0, 2, 10, FREQ, 1)) == 1
+    t.free()
     keys = ["input", "illustrations", "illustration"]
-    t = _tree_of(R, keys)
+    t = _RefTree(ref, keys)
     for k in keys:
-        assert len(_both(R, am, t, k, 0, 0, 10, FREQ, 1)) == (2 if k == "illustration" else 1)
-        assert _both(R, am, t, k, 0, 0, 10, FREQ, 0) == [k]
-    R.ref_art_free(t)
+        assert len(_both(ref, am, t, k, 0, 0, 10, FREQ, 1)) == (2 if k == "illustration" else 1)
+        assert _both(ref, am, t, k, 0, 0, 10, FREQ, 0) == [k]
+    t.free()
     # test_art_search_sku_like_tokens :914 and test_art_search_ill_like_tokens :964 (test/skus.txt, test/ill.txt: byte copies in tests/golden)
     skus = [l.rstrip("\n") for l in open(os.path.join(ROOT, "tests", "golden", "art_skus.txt"))]
-    t = _tree_of(R, skus)
+    t = _RefTree(ref, skus)
     for k in skus:
-        assert _both(R, am, t, k, 0, 0, 10, FREQ, 1) == [k]
-        assert _both(R, am, t, k, 0, 0, 10, FREQ, 0) == [k]
-    R.ref_art_free(t)
+        assert _both(ref, am, t, k, 0, 0, 10, FREQ, 1) == [k]
+        assert _both(ref, am, t, k, 0, 0, 10, FREQ, 0) == [k]
+    t.free()
     ill = [l.rstrip("\n") for l in open(os.path.join(ROOT, "tests", "golden", "art_ill.txt"))]
     counts = {"input": 2, "illustration": 2, "image": 7, "instrument": 2, "in": 10, "info": 2, "inventor": 2, "imageresize": 2, "id": 5,
               "insect": 2, "ice": 2}
-    t = _tree_of(R, ill)
+    t = _RefTree(ref, ill)
     for k in ill:
-        got = _both(R, am, t, k, 0, 0, 10, FREQ, 1)
+        got = _both(ref, am, t, k, 0, 0, 10, FREQ, 1)
         assert len(got) == counts.get(k, 1) and (k in counts or got == [k]), (k, got)
-        assert _both(R, am, t, k, 0, 0, 10, FREQ, 0) == [k]
-    R.ref_art_free(t)
+        assert _both(ref, am, t, k, 0, 0, 10, FREQ, 0) == [k]
+    t.free()
 
 
 def test_device_walk_function_equals_the_host_walk(am):

@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 import oracle_lib as ol
 
 ROOT = ol.ROOT
@@ -46,3 +48,36 @@ def test_product_arm_needs_cuda():
     r = run(SMALL)
     assert r.returncode != 0 and r.stdout.strip() == ""
     assert "no CPU fallback" in r.stderr
+
+
+def _dumped(d):
+    import numpy as np
+    files = sorted(os.listdir(d))
+    arrays = {f: np.load(os.path.join(d, f)) for f in files}
+    assert "count.npy" in arrays and "key.npy" in arrays
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(os.path.getsize(os.path.join(d, f)) for f in files) <= 64 << 20
+    return arrays
+
+
+def _same_outputs(args, n_queries, tmp_path):
+    import numpy as np
+    runs = []
+    for i in range(2):
+        r = run(args + ["--dump-outputs", str(tmp_path / str(i))])
+        assert r.returncode == 0, r.stderr[-2000:]
+        runs.append(_dumped(tmp_path / str(i)))
+    assert runs[0].keys() == runs[1].keys()
+    for f in runs[0]:
+        assert np.array_equal(runs[0][f], runs[1][f]), f
+    n = runs[0]["count.npy"]
+    assert len(n) == n_queries and n.sum() > 0 and (runs[0]["key.npy"][:, :int(n.max())] != 0).any()
+
+
+def test_reference_arm_dumps_the_same_outputs_every_run(tmp_path):
+    _same_outputs(["--impl", "reference"] + SMALL, 32, tmp_path)
+
+
+@pytest.mark.gpu
+def test_product_arm_dumps_the_same_outputs_every_run(tmp_path):
+    _same_outputs(SMALL + ["--no-cpu-baseline", "--no-other-configs", "--no-graph-cache", "--recall-queries", "0"], 64, tmp_path)

@@ -20,6 +20,7 @@ GPU_ONLY = [
     "tests/test_gpu_parity.py::test_knn_selective_filters_long_walks",            # builds its graph on the device, asserts device counters
     "tests/test_gpu_parity.py::test_hnsw_load_rejects_malformed_graph_and_keeps_the_old_one",   # asserts the library's load-time validation
     "tests/test_incremental_mirror.py::test_append_lists_rejects_malformed_input",              # asserts the library's argument validation
+    "tests/test_bench_contract.py::test_product_arm_dumps_the_same_outputs_every_run",          # runs bench.py's CUDA arm in a subprocess
 ]
 
 

@@ -125,7 +125,6 @@ def test_append_lists_rejects_malformed_input():
     gi.close()
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built (reference tree absent)")
 @pytest.mark.skipif(__import__("os").environ.get("TSGPU_TEST_DOUBLE") != "1",
                     reason="a check of the DATA PATH reference posting_list_t -> mirror: runs in the dry run against the oracle double "
                            "(tests/test_gpu_tests_dryrun.py); the device side of the same calls is test_patched_mirror_equals_fresh_mirror")
@@ -133,15 +132,22 @@ def test_mirror_follows_the_reference_posting_lists():
     """The write side as the reference keeps it: one posting_list_t per token — the reference's OWN src/posting_list.cpp, compiled in
     oracle/_ref — receives posting_t::upsert / erase for every written document; after each batch of writes the touched tokens' lists
     are read back through the reference's iterator (what the binding of INTEGRATION.md §1 does) and handed to tsgpu_index_append_lists.
-    The patched mirror must answer exactly like the oracle over the reference's lists as they stand."""
+    The patched mirror must answer exactly like the oracle over the reference's lists as they stand. Each list read back must equal
+    the list the writes describe, which is what the mirror is loaded with; without oracle/_ref that equality is checked against the
+    reference's answers stored in tests/golden/ref_answers (oracle_lib.RefAnswers)."""
+    with ol.RefAnswers("test_incremental_mirror", "reference_posting_lists") as ref:
+        _mirror_follows_the_reference_posting_lists(ref)
+
+
+def _mirror_follows_the_reference_posting_lists(ref):
     import ctypes as C
-    R = ol.ref()
+    R = ol.ref() if ref.live else None
     rng = np.random.default_rng(11)
     vocab, n_docs = 80, 3000
     zipf = np.arange(1, vocab + 1, dtype=np.float64) ** -1.0
     zipf /= zipf.sum()
-    plists = [C.c_void_p(R.ref_plist_new(256)) for _ in range(vocab)]
-    doc_tokens = {}
+    plists = [C.c_void_p(R.ref_plist_new(256)) for _ in range(vocab)] if ref.live else None
+    doc_tokens, doc_offsets = {}, {}
 
     def offsets_of(tokens):
         """Index::tokenize_string (src/index.cpp:1323-1349): 1-based positions per token, a trailing 0 on the document's last token"""
@@ -154,21 +160,32 @@ def test_mirror_follows_the_reference_posting_lists():
     def write(doc, tokens, touched):
         if doc in doc_tokens:                                   # an update: Index::remove_field first
             for t in offsets_of(doc_tokens[doc]):
-                R.ref_plist_erase(plists[t], doc); touched.add(t)
+                if ref.live:
+                    R.ref_plist_erase(plists[t], doc)
+                touched.add(t)
         if tokens is None:
             doc_tokens.pop(doc, None)
+            doc_offsets.pop(doc, None)
             return
         for t, offs in offsets_of(tokens).items():
             a = np.asarray(offs, np.uint32)
-            R.ref_plist_upsert(plists[t], doc, ol.p32(a), len(a)); touched.add(t)
+            if ref.live:
+                R.ref_plist_upsert(plists[t], doc, ol.p32(a), len(a))
+            touched.add(t)
         doc_tokens[doc] = tokens
+        doc_offsets[doc] = offsets_of(tokens)
 
-    def dump(t):
+    def read_back(t):
         n = R.ref_plist_num_ids(plists[t])
         ids = np.zeros(n + 1, np.uint32); oi = np.zeros(n + 2, np.uint32); offs = np.zeros(8 * n + 16, np.uint32)
         k = R.ref_plist_dump(plists[t], ol.p32(ids), ol.p32(oi), ol.p32(offs), len(ids), len(offs))
         assert k == n
         return [(int(ids[i]), offs[int(oi[i]):int(oi[i + 1])].tolist()) for i in range(n)]
+
+    def dump(t):
+        want = [(d, per[t]) for d, per in sorted(doc_offsets.items()) if t in per]
+        assert ref.same(want, lambda: read_back(t)), t
+        return want
 
     def random_doc():
         return rng.choice(vocab, int(rng.integers(2, 7)), p=zipf).tolist()
@@ -219,6 +236,7 @@ def test_mirror_follows_the_reference_posting_lists():
         for k, t in enumerate(part):
             remap[t] = first + k
         check(10 + batch)
-    for h in plists:
-        R.ref_plist_free(h)
+    if ref.live:
+        for h in plists:
+            R.ref_plist_free(h)
     gi.close()
